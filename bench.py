@@ -27,6 +27,7 @@ import argparse
 import json
 import os
 import sys
+import tempfile
 import threading
 import time
 
@@ -34,6 +35,8 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+# the tree may be read-only: numba's compiled-function cache (synth.py) goes to a temporary directory
+os.environ.setdefault("NUMBA_CACHE_DIR", os.path.join(tempfile.gettempdir(), f"superodom_b200_numba_cache_{os.getuid()}"))
 
 METRIC = "ICP scans/sec (128-beam, 1M-pt map)"
 UNIT = "scans/s"
@@ -45,6 +48,7 @@ KNN_BYTES_PER_QUERY = 16 + 5 * 8
 # ncu --set full, dram__bytes_read.sum + dram__bytes_write.sum of ONE k_knn_scan launch / its queries (profiles/README.md says
 # which capture; None where no capture of the current kernel is committed)
 NCU_DRAM_BYTES_PER_QUERY = {"k_knn_scan": 76.8, "k_knn_fit": None}      # profiles/ncu_prof_r2t_metrics.csv: (26.78 MB read + 53.74 MB written) / 1 048 576 queries
+DUMP_MAX_BYTES = 64 << 20
 
 
 def _peaks():
@@ -184,6 +188,25 @@ def cfg5_queries(map_xyzi: np.ndarray, first: int, count: int, block: int = 125_
     return out
 
 
+def dump_outputs(out_dir, results, **extra):
+    """Write what the last timed step returned as out_dir/<name>.npy (float64): one row per scan, scans in call order, for every
+    field of the result struct except the timings and padding, plus `extra` arrays.  Above DUMP_MAX_BYTES a fixed (seed 0) sample
+    of the scans is written; scan_index.npy names the scans of the rows either way."""
+    fields = [f for f, _ in type(results[0])._fields_ if not f.startswith("time_") and not f.endswith("_")]
+    per_scan = {f: np.array([np.asarray(getattr(r, f), dtype=np.float64).reshape(-1) for r in results]) for f in fields}
+    index = np.arange(len(results))
+    budget = DUMP_MAX_BYTES - sum(np.asarray(a).nbytes for a in extra.values())
+    row_bytes = sum(a.shape[1] * 8 for a in per_scan.values()) + 8
+    if len(results) * row_bytes > budget:
+        index = np.sort(np.random.default_rng(0).choice(len(results), max(0, budget // row_bytes), replace=False))
+    arrays = {f: (a[index, 0] if a.shape[1] == 1 else a[index]) for f, a in per_scan.items()}
+    arrays["scan_index"] = index
+    arrays.update(extra)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 # ----------------------------------------------------------------------------------------------------------------
 def run_reference(args):
     """The reference's CPU implementation of the path on the host cores: oracle/_ref (reference octree.h compiled
@@ -201,15 +224,17 @@ def run_reference(args):
     mode = 2 if ref else 0
 
     def step():
-        for s, p in zip(scans, priors):
-            r = om.register(s, p, 0.2, 20, 0, knn_mode=mode, n_threads=cores, skip_map_checks=True)
-            assert r.status == 0
+        res = [om.register(s, p, 0.2, 20, 0, knn_mode=mode, n_threads=cores, skip_map_checks=True) for s, p in zip(scans, priors)]
+        assert all(r.status == 0 for r in res)
+        return res
     for _ in range(args.warmup):
         step()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        step()
+        res = step()
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, res)
     v = sample * args.steps / dt
     kind = "reference-octree+port" if ref else "port"
     line = {"impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
@@ -351,6 +376,8 @@ def run_ours(args):
     if sampler:
         sampler.close()
     launches = ctx.kernel_launches()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, [r for rk in res for r in rk], gathered_rows=gathered.cpu().numpy())
     n_total = per_step * world
     value = n_total * args.steps / (ms * 1e-3)
 
@@ -672,7 +699,10 @@ def main():
     ap.add_argument("--no-cfg4", action="store_true")
     ap.add_argument("--no-cfg5", action="store_true")
     ap.add_argument("--no-live", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the per-scan results of the last step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

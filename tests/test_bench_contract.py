@@ -5,13 +5,15 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def test_reference_arm_prints_one_json_line():
+def test_reference_arm_prints_one_json_line(tmp_path):
     env = dict(os.environ, SO_BENCH_CACHE="")                       # no cache side effects from the test suite
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "1", "--steps", "1", "--warmup", "0",
-                          "--ref-scans", "1"], capture_output=True, text=True, env=env, timeout=600)
+                          "--ref-scans", "1", "--dump-outputs", str(tmp_path / "out")], capture_output=True, text=True, env=env, timeout=600)
     assert out.returncode == 0, out.stderr[-2000:]
     lines = [ln for ln in out.stdout.splitlines() if ln.strip()]
     assert len(lines) == 1, lines
@@ -21,6 +23,10 @@ def test_reference_arm_prints_one_json_line():
         assert k in d, k
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0 and d["e2e"]["value"] == d["value"]
     assert d["cpu_baseline"]["cores"] >= 1 and "workload" in d["config"]
+    # --dump-outputs: the last step's per-scan results, float64, one row per scan
+    pose, status = np.load(tmp_path / "out" / "pose.npy"), np.load(tmp_path / "out" / "status.npy")
+    assert pose.dtype == np.float64 and pose.shape == (1, 7) and abs(np.linalg.norm(pose[0, 3:]) - 1) < 1e-9
+    assert status.tolist() == [0.0] and np.load(tmp_path / "out" / "cov.npy").shape == (1, 36)
 
 
 def test_reference_arm_non_zero_ranks_exit_quietly():

@@ -4,11 +4,12 @@ Bars (task section 3): bit-exact for integer / index work (neighbour ids, float 
 iteration counts); FP64 quantities within the stated tolerances (normal equations 1e-10 relative, pose 1e-4 m /
 1e-4 rad per BASELINE.json north_star -- observed ~1e-15)."""
 import ctypes as C
+import os
 
 import numpy as np
 import pytest
 
-from conftest import get_case, quat_angle
+from conftest import GOLDEN, get_case, hall_queries, quat_angle, reference_knn, reference_registration
 
 pytestmark = pytest.mark.gpu
 
@@ -39,10 +40,7 @@ def test_knn_bit_exact(gpu_api, oracle_mod, name):
     case = get_case(name)
     ctx = _ctx(gpu_api, case)
     om = oracle_mod.OracleMap(case["map_xyzi"])
-    rng = np.random.default_rng(0)
-    base = case["map_xyzi"][::7, :3]
-    q = base + rng.normal(0, 0.12, size=base.shape).astype(np.float32)
-    q = np.concatenate([q, rng.uniform(-30, 30, size=(500, 3)).astype(np.float32) + q.mean(0)])     # incl. far-away queries
+    q = hall_queries(case["map_xyzi"])                    # incl. far-away queries
     gi, gd = ctx.knn(q, 5, 0.0)                           # exact, unbounded
     oi, od, of = om.knn(q, 5, 0)
     assert np.array_equal(_gi(gi)[of], oi[of]) and np.array_equal(gd[of], od[of])
@@ -56,8 +54,8 @@ def test_knn_bit_exact(gpu_api, oracle_mod, name):
         gi, gd = ctx.knn(q[:2000], k, 0.0)
         oi, od, of = om.knn(q[:2000], k, 0)
         assert np.array_equal(_gi(gi)[of], oi[of]) and np.array_equal(gd[of], od[of])
-    if name == "hall" and oracle_mod.has_ref_octree():    # reference's own octree (verbatim) agrees here
-        ri, rd, rf = om.knn(q[:-500], 5, 2)
+    if name == "hall":                                    # reference's own octree (stored outputs) agrees here
+        ri, rd = reference_knn("hall_knn", om, q[:-500])
         gi, gd = ctx.knn(q[:-500], 5, 0.0)
         assert np.array_equal(_gi(gi), ri) and np.array_equal(gd, rd)
     ctx.close()
@@ -125,17 +123,16 @@ def test_register_pose_parity(gpu_api, oracle_mod, name, cap):
     assert np.linalg.norm(np.array(r.pose)[:3] - case["pose_true"][:3]) < 0.02
     r2 = ctx.register(case["scan_xyzi"], case["pose_prior"], cfg["max_iterations"], cap)
     assert np.array_equal(np.array(r.pose), np.array(r2.pose)) and np.array_equal(np.array(r.cov), np.array(r2.cov))
-    if name == "hall" and oracle_mod.has_ref_octree():
-        # the reference's own (verbatim) octree in the loop: same pose, because on this layout the octree is exact
-        rr = om.register(case["scan_xyzi"], case["pose_prior"], cfg["plane_res"], cfg["max_iterations"], cap, knn_mode=2)
+    if name == "hall":
+        # the reference's own octree in the loop (stored run): same pose, because on this layout the octree is exact
+        rr, _, _ = reference_registration("hall", om, case["scan_xyzi"], case["pose_prior"], cfg, cap)
         _assert_pose_close(np.array(r.pose), np.array(rr.pose))
         assert rr.n_iterations == r.n_iterations
     ctx.close()
 
 
-def test_golden_fixture_through_the_abi(gpu_api):
-    import os
-    G = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "tiny_case.npz"))
+def test_golden_fixture_through_the_abi(gpu_api, oracle_mod):
+    G = np.load(os.path.join(GOLDEN, "tiny_case.npz"))
     ctx = gpu_api.Context(max_map_points=1 << 20, max_scan_points=65536, plane_res=float(G["plane_res"]))
     ctx.map_set_points(G["map_xyzi"])
     gc, gho, ghr = ctx.correspond(G["scan_xyzi"], G["pose_prior"], 0)
@@ -148,6 +145,11 @@ def test_golden_fixture_through_the_abi(gpu_api):
     r = ctx.register(G["scan_xyzi"], G["pose_prior"], int(G["max_iterations"]), 0)
     _assert_pose_close(np.array(r.pose), G["pose_exact"])
     assert r.n_iterations == int(G["n_iterations_exact"])
+    # the reference octree's neighbour sets injected after the search reproduce its registration of the fixture
+    rr, trace, _ = reference_registration("golden_tiny", oracle_mod.OracleMap(G["map_xyzi"]), G["scan_xyzi"], G["pose_prior"],
+                                          {"plane_res": float(G["plane_res"])}, 0)
+    ri = ctx.register_injected(G["scan_xyzi"], G["pose_prior"], int(G["max_iterations"]), trace, 0)
+    assert ri.n_iterations == rr.n_iterations and np.abs(np.array(ri.pose) - G["pose_ref_octree"]).max() <= 1e-9
     ctx.close()
 
 

@@ -1,14 +1,12 @@
 """CPU tests of the oracle itself: its small linear algebra against numpy, its k-NN modes against each other and
-against the reference's own octree (compiled verbatim into oracle/_ref), its Ceres-style solver against first
-principles, and the committed golden fixtures."""
+against stored outputs of the reference's own octree (tests/golden/reference_octree.npz), its Ceres-style solver against
+first principles, and the committed golden fixtures."""
 import os
 
 import numpy as np
 import pytest
 
-from conftest import get_case, quat_angle
-
-GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+from conftest import GOLDEN, get_case, octree_pin_queries, quat_angle, reference_knn, reference_registration, x_dominant_map
 
 
 def test_sym_eig_and_qr_against_numpy(oracle_mod):
@@ -90,39 +88,21 @@ def test_knn_exact_equals_brute_force(oracle_mod):
         assert np.array_equal(order, i0[j]) and np.array_equal(d2[order], d0[j])
 
 
-def _x_dominant_map():
-    """Block-local cloud with a dominant x extent and x, y, z value ranges far apart: the layout on which the
-    reference octree's two bugs (flann/octree.h:383-385 bbox, :984-1001 inside()) cannot fire."""
-    rng = np.random.default_rng(11)
-    n = 40000
-    x = rng.uniform(77.0, 123.0, n)
-    y = rng.uniform(-9.0, 9.0, n)
-    z = np.where(rng.uniform(size=n) < 0.5, -1.8, rng.uniform(-1.8, 5.0, n))
-    y = np.where(rng.uniform(size=n) < 0.3, np.round(y / 4.5) * 4.5, y)
-    p = np.stack([x, y, z], 1) + rng.normal(0, 0.02, size=(n, 3))
-    return np.concatenate([p, np.ones((n, 1))], 1).astype(np.float32)
-
-
 def test_reference_octree_pins_the_knn_restatement(oracle_mod):
     """Parity pin for SURVEY 8(c): where the verbatim reference octree is exact, the oracle's exact k-NN must equal
     it bit for bit (indices AND float distances).  Elsewhere the mismatch rate is reported."""
     O = oracle_mod
-    if not O.has_ref_octree():
-        pytest.skip("oracle/_ref not built (no /root/reference on this box and no prebuilt _ref)")
-    xyzi = _x_dominant_map()
-    m = O.OracleMap(xyzi)
-    rng = np.random.default_rng(2)
-    q = xyzi[::13, :3] + rng.normal(0, 0.1, size=xyzi[::13, :3].shape).astype(np.float32)
-    i0, d0, _ = m.knn(q, 5, 0)
-    i2, d2, _ = m.knn(q, 5, 2)
+    xyzi, cfg1_map = x_dominant_map(), get_case("cfg1")["map_xyzi"]
+    qx, q = octree_pin_queries(xyzi, cfg1_map)
+    m = O.OracleMap(xyzi, ref_octree=False)
+    i0, d0, _ = m.knn(qx, 5, 0)
+    i2, d2 = reference_knn("x_dominant", m, qx)
     assert np.array_equal(d0, d2)
     assert np.array_equal(i0, i2)
     # on the warehouse scene the octree is NOT exact (two reference bugs): report, and bound, the rate
-    c = get_case("cfg1")
-    m = O.OracleMap(c["map_xyzi"])
-    q = c["map_xyzi"][::37, :3] + rng.normal(0, 0.1, size=c["map_xyzi"][::37, :3].shape).astype(np.float32)
+    m = O.OracleMap(cfg1_map, ref_octree=False)
     i0, d0, _ = m.knn(q, 5, 0)
-    i2, d2, _ = m.knn(q, 5, 2)
+    i2, d2 = reference_knn("cfg1_knn", m, q)
     bad = int((np.sort(i0, 1) != np.sort(i2, 1)).any(1).sum())
     print(f"reference octree vs exact on cfg1 warehouse: {bad}/{len(q)} queries differ")
     assert bad < 0.02 * len(q)
@@ -224,11 +204,11 @@ def test_map_shift_rolls_origin(oracle_mod):
 
 def test_golden_fixtures(oracle_mod):
     """Fixtures were generated by tests/golden/make_golden.py from the oracle/_ref build (reference octree in the loop).
-    They pin the oracle against regressions; they are NOT reference outputs (the reference ships none, SURVEY section 4)."""
+    They pin the oracle against regressions; they are NOT reference outputs (the reference ships none, SURVEY section 4).
+    The octree-in-the-loop run of the same fixture is stored in reference_octree.npz: its per-iteration neighbour sets must
+    be rebuilt from this oracle's exact search (and its pose is the fixture's pose_ref_octree)."""
     O = oracle_mod
     path = os.path.join(GOLDEN, "tiny_case.npz")
-    if not os.path.exists(path):
-        pytest.skip("golden fixture missing")
     G = np.load(path)
     m = O.OracleMap(G["map_xyzi"])
     corr, ho, hr = m.correspond(G["scan_xyzi"], G["pose_prior"], float(G["plane_res"]), 0, 0)
@@ -243,9 +223,8 @@ def test_golden_fixtures(oracle_mod):
     r = m.register(G["scan_xyzi"], G["pose_prior"], float(G["plane_res"]), int(G["max_iterations"]), 0, knn_mode=0)
     assert np.allclose(np.array(r.pose), G["pose_exact"], atol=1e-9)
     assert r.n_iterations == int(G["n_iterations_exact"])
-    if O.has_ref_octree():
-        r2 = m.register(G["scan_xyzi"], G["pose_prior"], float(G["plane_res"]), int(G["max_iterations"]), 0, knn_mode=2)
-        assert np.allclose(np.array(r2.pose), G["pose_ref_octree"], atol=1e-9)
+    r2, _, _ = reference_registration("golden_tiny", m, G["scan_xyzi"], G["pose_prior"], {"plane_res": float(G["plane_res"])}, 0)
+    assert np.array_equal(np.array(r2.pose), G["pose_ref_octree"])
 
 
 # ---------------------------------------------------------------------------------------------------------------

@@ -7,10 +7,12 @@ from hypothesis import given, settings, strategies as st
 from hypothesis.extra import numpy as hnp
 
 finite = st.floats(min_value=-50.0, max_value=50.0, allow_nan=False, allow_infinity=False, width=64)
+# the plane fit solves on map points, which are float32: entries whose squares underflow in double (|x| < 1e-154) never reach it
+point_coords = st.floats(min_value=-50.0, max_value=50.0, allow_nan=False, allow_infinity=False, width=32)
 
 
 @settings(max_examples=60, deadline=None)
-@given(hnp.arrays(np.float64, (5, 3), elements=finite))
+@given(hnp.arrays(np.float64, (5, 3), elements=point_coords))
 def test_colpiv_qr_matches_lstsq_when_well_conditioned(oracle_mod, A):
     b = -np.ones(5)
     s = np.linalg.svd(A, compute_uv=False)

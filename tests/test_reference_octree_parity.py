@@ -1,5 +1,8 @@
 """Parity against the reference's REAL k-NN path: nanoflann::Octree::knnNeighbors (flann/octree.h:1004-1055, called from
-LocalMap::nearestKSearchSurf, LocalMap.h:509-521), compiled verbatim into oracle/_ref, on the BASELINE configurations.
+LocalMap::nearestKSearchSurf, LocalMap.h:509-521), on the BASELINE configurations.  Its outputs come from
+tests/golden/reference_octree.npz, written by tests/golden/make_reference_octree.py with the octree compiled verbatim into the
+oracle (conftest.reference_registration rebuilds them and checks their SHA-256).  The cfg2 / cfg3 scans are taken every 8th
+point (conftest.OCTREE_CASES) so that the stored neighbour rows stay small.
 
 The reference octree is not an exact k-NN (`inside()` tests x on all three axes, the root bbox update compares x against
 the y/z maxima and writes min[2] for max[2]: octree.h:383-385,984-1001); this library searches exactly inside the block
@@ -10,20 +13,19 @@ the y/z maxima and writes min[2] for max[2]: octree.h:383-385,984-1001); this li
       within the north-star tolerance (1e-4 m / 1e-4 rad; observed ~1e-12).  Hence the k-NN is the ONLY deviation.
   (B) BOUND: the deviation the exact search causes -- GPU exact vs octree-in-the-loop -- is recorded (mismatching queries,
       |dpos|, |drot|) and bounded (<= 5e-4 m / 5e-4 rad), and the exact result is not farther from ground truth than the
-      octree result beyond that bound.  The numbers are written to gpurun_out/octree_parity.json and printed.
+      octree result beyond that bound.  The numbers are printed.
 """
 import json
-import os
 
 import numpy as np
 import pytest
 
-from conftest import get_case, quat_angle
+from conftest import OCTREE_CASES, get_case, quat_angle, reference_registration
 
 pytestmark = pytest.mark.gpu
 
-CASES = [("cfg1", 2000), ("cfg1", 0), ("cfg2", 0), ("cfg3", 0)]
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+CASES = [(name, cap) for name, cap, _ in OCTREE_CASES]
+STRIDE = {(name, cap): stride for name, cap, stride in OCTREE_CASES}
 
 
 def _ctx(api, case):
@@ -33,36 +35,24 @@ def _ctx(api, case):
 
 
 def _record(key, row):
-    out = os.path.join(ROOT, "gpurun_out")
-    try:
-        os.makedirs(out, exist_ok=True)
-        path = os.path.join(out, "octree_parity.json")
-        data = {}
-        if os.path.exists(path):
-            with open(path) as f:
-                data = json.load(f)
-        data[key] = row
-        with open(path, "w") as f:
-            json.dump(data, f, indent=1, sort_keys=True)
-    except OSError:
-        pass
     print(f"[octree-parity] {key}: {json.dumps(row)}")
+
+
+def _reference(oracle_mod, name, cap):
+    case = get_case(name)
+    scan = case["scan_xyzi"][::STRIDE[(name, cap)]]
+    om = oracle_mod.OracleMap(case["map_xyzi"], ref_octree=False)
+    ro, trace, status = reference_registration(f"{name}_cap{cap}", om, scan, case["pose_prior"], case["cfg"], cap)
+    return case, scan, om, ro, trace, status
 
 
 @pytest.mark.parametrize("name,cap", CASES)
 def test_injected_reference_octree_neighbours_reproduce_the_reference_path(gpu_api, oracle_mod, name, cap):
-    if not oracle_mod.has_ref_octree():
-        pytest.skip("oracle/_ref (reference octree compiled verbatim) not present")
-    case = get_case(name)
-    cfg = case["cfg"]
-    scan, prior = case["scan_xyzi"], case["pose_prior"]
-    om = oracle_mod.OracleMap(case["map_xyzi"], ref_octree=True)
-    trace = np.zeros((cfg["max_iterations"], len(scan), 5), np.int64)
-    ro = om.register(scan, prior, cfg["plane_res"], cfg["max_iterations"], cap, knn_mode=2, n_threads=8, nn_trace=trace)
-    assert ro.status == 0
+    case, scan, om, ro, trace, _ = _reference(oracle_mod, name, cap)
+    cfg, prior = case["cfg"], case["pose_prior"]
     n = ro.n_iterations
     ctx = _ctx(gpu_api, case)
-    r = ctx.register_injected(scan, prior, cfg["max_iterations"], trace[:n], cap)
+    r = ctx.register_injected(scan, prior, cfg["max_iterations"], trace, cap)
     assert r.status == 0
     # (A) identical control flow and counts, pose far inside the tolerance
     assert r.n_iterations == n
@@ -84,26 +74,20 @@ def test_injected_reference_octree_neighbours_reproduce_the_reference_path(gpu_a
 
 @pytest.mark.parametrize("name,cap", CASES)
 def test_exact_knn_deviation_from_reference_octree_is_bounded(gpu_api, oracle_mod, name, cap):
-    if not oracle_mod.has_ref_octree():
-        pytest.skip("oracle/_ref (reference octree compiled verbatim) not present")
-    case = get_case(name)
-    cfg = case["cfg"]
-    scan, prior, truth = case["scan_xyzi"], case["pose_prior"], case["pose_true"]
-    om = oracle_mod.OracleMap(case["map_xyzi"], ref_octree=True)
-    ro = om.register(scan, prior, cfg["plane_res"], cfg["max_iterations"], cap, knn_mode=2, n_threads=8)      # reference octree in the loop
+    case, scan, om, ro, trace, status2 = _reference(oracle_mod, name, cap)                                  # reference octree in the loop
+    cfg, prior, truth = case["cfg"], case["pose_prior"], case["pose_true"]
     ctx = _ctx(gpu_api, case)
     r = ctx.register(scan, prior, cfg["max_iterations"], cap)                                                # exact in-block k-NN
-    assert r.status == 0 and ro.status == 0
+    assert r.status == 0
     pg, po = np.array(r.pose), np.array(ro.pose)
     dpos, drot = float(np.linalg.norm(pg[:3] - po[:3])), float(quat_angle(pg[3:], po[3:]))
     eg = float(np.linalg.norm(pg[:3] - truth[:3]))
     eo = float(np.linalg.norm(po[:3] - truth[:3]))
     # mismatch rate of the neighbour sets at the prior pose (first ICP iteration)
-    oc2, _, _ = om.correspond(scan, prior, cfg["plane_res"], cap, 2, n_threads=8)
     oc0, _, _ = om.correspond(scan, prior, cfg["plane_res"], cap, 0, n_threads=8)
     searched = (oc0["status"] >= 0) & (oc0["status"] != 1)
-    mism = searched & (np.sort(oc2["nn"], 1) != np.sort(oc0["nn"], 1)).any(1)
-    gates = searched & (oc2["status"] != oc0["status"])
+    mism = searched & (np.sort(trace[0], 1) != np.sort(oc0["nn"], 1)).any(1)
+    gates = searched & (status2 != oc0["status"])
     row = {"queries": int(searched.sum()), "octree_wrong_neighbour_sets": int(mism.sum()), "mismatch_rate": float(mism.sum() / max(1, searched.sum())),
            "gate_flips": int(gates.sum()), "dpos_gpu_exact_vs_octree_m": dpos, "drot_rad": drot, "err_vs_truth_gpu_exact_m": eg,
            "err_vs_truth_octree_m": eo, "icp_iterations_gpu": int(r.n_iterations), "icp_iterations_octree": int(ro.n_iterations)}
