@@ -114,7 +114,7 @@ __device__ __noinline__ void covariance_and_errors(IcpState& st) {
 // round-robin order of jacobi_eig6_rr: the three angles of a round are computed by three lanes at once, and each rotation updates
 // its 8 off-diagonal entries, 12 eigenvector entries and 2x2 block on 15 lanes in one step instead of ~110 dependent FP64
 // instructions on one thread (the covariance was 38 of the ~50 us the last optimiser step of a registration took).  Per element
-// the arithmetic and its order are those of the serial routine.
+// the arithmetic and its order are those of the serial routine; the 2x2 block goes through the same jacobi_rot2.
 __constant__ int c_rr_p[15] = {0, 1, 2, 0, 3, 1, 0, 2, 1, 0, 1, 4, 0, 2, 3};
 __constant__ int c_rr_q[15] = {5, 4, 3, 4, 5, 2, 3, 4, 5, 2, 3, 5, 1, 5, 4};
 struct CovScratch { double a[36], v[36], w[6], inv[6], t[3], c[3], s[3]; int perm[6]; };
@@ -163,14 +163,14 @@ __device__ __noinline__ void covariance_and_errors_warp(IcpState& S, CovScratch&
                     // lanes 0..5: row r of a (r outside the pair); lanes 8..13: row r of v; lane 16: the 2x2 block
                     const int r = lane < 8 ? lane : lane - 8;
                     const bool do_a = lane < 6 && r != p && r != q, do_v = lane >= 8 && lane < 14, do_d = lane == 16;
-                    double n0 = 0.0, n1 = 0.0;
+                    double n0 = 0.0, n1 = 0.0, n2 = 0.0;
                     if (do_a) { const double arp = sc.a[r * 6 + p], arq = sc.a[r * 6 + q]; n0 = c * arp - sn * arq; n1 = sn * arp + c * arq; }
                     if (do_v) { const double vrp = sc.v[r * 6 + p], vrq = sc.v[r * 6 + q]; n0 = c * vrp - sn * vrq; n1 = sn * vrp + c * vrq; }
-                    if (do_d) { const double apq = sc.a[p * 6 + q]; n0 = sc.a[p * 6 + p] - t * apq; n1 = sc.a[q * 6 + q] + t * apq; }
+                    if (do_d) jacobi_rot2(sc.a[p * 6 + p], sc.a[q * 6 + q], sc.a[p * 6 + q], c, sn, n0, n1, n2);
                     __syncwarp();
                     if (do_a) { sc.a[r * 6 + p] = sc.a[p * 6 + r] = n0; sc.a[r * 6 + q] = sc.a[q * 6 + r] = n1; }
                     if (do_v) { sc.v[r * 6 + p] = n0; sc.v[r * 6 + q] = n1; }
-                    if (do_d) { sc.a[p * 6 + p] = n0; sc.a[q * 6 + q] = n1; sc.a[p * 6 + q] = 0.0; sc.a[q * 6 + p] = 0.0; }
+                    if (do_d) { sc.a[p * 6 + p] = n0; sc.a[q * 6 + q] = n1; sc.a[p * 6 + q] = n2; sc.a[q * 6 + p] = n2; }
                     __syncwarp();
                 }
             }

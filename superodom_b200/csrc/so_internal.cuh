@@ -126,6 +126,19 @@ __host__ __device__ inline void rel_motion(const double a[7], const double b[7],
 #ifndef SO_JACOBI_OFF_TOL
 #define SO_JACOBI_OFF_TOL 1e-33
 #endif
+// The 2x2 block [app apq; apq aqq] after one rotation J = [c s; -s c]: the exact similarity J^T A J of the (c, s) actually used.
+// The angle comes from an FP32 tangent, so the classic shortcut app -= t apq, aqq += t apq, apq = 0 -- exact only for the exact
+// root t -- would perturb the matrix by ~1e-7 |apq| per rotation (eigenvalue error ~1e-8 cond, direction error up to 5e-8).  With
+// the exact update the inexact angle only leaves a ~1e-7 |apq| off-diagonal for the next sweep to remove.  Explicit roundings:
+// the serial and warp covariance routines produce the same bits from it.
+__device__ __forceinline__ void jacobi_rot2(double app, double aqq, double apq, double c, double s, double& npp, double& nqq, double& npq) {
+    const double cc = __dmul_rn(c, c), ss = __dmul_rn(s, s), cs = __dmul_rn(c, s);
+    const double x = __dmul_rn(2.0 * cs, apq);
+    npp = __fma_rn(ss, aqq, __fma_rn(cc, app, -x));
+    nqq = __fma_rn(ss, app, __fma_rn(cc, aqq, x));
+    npq = __fma_rn(cs, __dsub_rn(app, aqq), __dmul_rn(__dsub_rn(cc, ss), apq));
+}
+
 template <int N, int SWEEPS, bool WITH_V = true>
 __device__ inline void jacobi_eig(double* a, double* v, double* w) {
     if (WITH_V) {
@@ -153,14 +166,16 @@ __device__ inline void jacobi_eig(double* a, double* v, double* w) {
                     // tan of the rotation angle, t = sgn(theta) / (|theta| + sqrt(theta^2 + 1)), theta = (aqq - app) / (2 apq),
                     // evaluated in FP32 (one MUFU sqrt + one MUFU rcp instead of an FP64 sqrt and divide).  The rotation
                     // itself stays exactly orthogonal in FP64 because c = rsqrt(1 + t^2), s = t c are formed in FP64 from
-                    // whatever t is; a 1e-7-accurate t only leaves a 1e-7-times-smaller off-diagonal for the next sweep
-                    // (measured: 3.9 sweeps instead of 3.4 to reach 1e-16, same eigenvalues to 2e-15).
+                    // whatever t is, and jacobi_rot2 applies exactly that rotation to the 2x2 block, so a 1e-7-accurate t
+                    // only leaves a 1e-7-times-smaller apq for the next sweep.
                     const float dlt = float(a[q * N + q] - a[p * N + p]), b2 = float(2.0 * apq);
                     float tf = __fdividef(b2, fabsf(dlt) + sqrtf(fmaf(dlt, dlt, b2 * b2)));
                     if (!(fabsf(tf) <= 1.0f)) tf = 0.0f;             // b2 == 0 after the cast (or inf/nan): no rotation
                     const double t = double(dlt < 0.0f ? -tf : tf);
                     const double c = rsqrt(t * t + 1.0), s = t * c;
-                    a[p * N + p] -= t * apq; a[q * N + q] += t * apq; a[p * N + q] = 0.0; a[q * N + p] = 0.0;
+                    double npp, nqq, npq;
+                    jacobi_rot2(a[p * N + p], a[q * N + q], apq, c, s, npp, nqq, npq);
+                    a[p * N + p] = npp; a[q * N + q] = nqq; a[p * N + q] = npq; a[q * N + p] = npq;
 #pragma unroll
                     for (int r = 0; r < N; ++r) {
                         if (r != p && r != q) {
@@ -239,7 +254,9 @@ __device__ inline void jacobi_eig6_rr(double* a, double* v, double* w) {
                 const int p = PP[round * 3 + k], q = QQ[round * 3 + k];
                 const double t = tt[k], c = cc[k], sn = ss[k], apq = a[p * N + q];
                 if (t != 0.0) {
-                    a[p * N + p] -= t * apq; a[q * N + q] += t * apq; a[p * N + q] = 0.0; a[q * N + p] = 0.0;
+                    double npp, nqq, npq;
+                    jacobi_rot2(a[p * N + p], a[q * N + q], apq, c, sn, npp, nqq, npq);
+                    a[p * N + p] = npp; a[q * N + q] = nqq; a[p * N + q] = npq; a[q * N + p] = npq;
 #pragma unroll
                     for (int r = 0; r < N; ++r) {
                         if (r != p && r != q) {
